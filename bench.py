@@ -195,9 +195,10 @@ def run_reference(args, rank, world):
     cannot be compiled in this image) on the box's host cores, same workload/metric.
     One step = one sweep over a bounded sample of the workload (up to 1024 of its instances, fewer when an
     instance is expensive: the whole run stays near half a minute); the thread count is the faster of "every
-    hardware thread" and "half of them"; the figure is the MEDIAN of 5 timed repeats, each of
-    max(--steps, 0.7 s worth of) steps, so a single slow repeat (thread start-up, a noisy neighbour) does
-    not move it."""
+    hardware thread" and "half of them".  The timed window is exactly --steps sweeps.  With --ref-seconds S
+    (the product arm's cpu_baseline) it is sized by time instead: the figure is the MEDIAN of 5 timed repeats,
+    each of max(0.7 s, S / 5) worth of sweeps, so a single slow repeat (thread start-up, a noisy neighbour)
+    does not move it."""
     if rank != 0:
         return
     import numpy as np
@@ -208,7 +209,7 @@ def run_reference(args, rank, world):
     avail = len(os.sched_getaffinity(0)) if hasattr(os, "sched_getaffinity") else (os.cpu_count() or 1)
     allthr = max(orc.num_threads(), avail)
     # Bounded sample: a probe of one instance per thread gives the time of one "round"; the sample is as many
-    # rounds as keep 5 repeats x --steps sweeps near 25 s (C2: the cap of 1024 instances; C5: one or two rounds).
+    # rounds as keep 5 x --steps sweeps near 25 s (C2: the cap of 1024 instances; C5: one or two rounds).
     def make(nb_):
         a = [x.numpy() for x in synth_batch_torch(torch, nb_, HORIZON, NX, NU, "cpu", 1234, NC)]
         return orc.BatchedOracle(NX, NU, NC, NCT, NX, HORIZON, nb_, *a)
@@ -232,28 +233,32 @@ def run_reference(args, rank, world):
     while nw < max(args.warmup, 1) or tw < 1.5:
         dt = bo.sweep(MUEQ, reps=1, nthreads=threads)
         t1, tw, nw = min(t1, dt), tw + dt, nw + 1
-    repeat_s = max(0.7, args.ref_seconds / 5.0)
-    steps = max(args.steps if args.ref_seconds <= 0 else 1, int(repeat_s / max(t1, 1e-5)) + 1)
+    if args.ref_seconds > 0:
+        repeats = 5
+        steps = int(max(0.7, args.ref_seconds / 5.0) / max(t1, 1e-5)) + 1
+    else:
+        repeats, steps = 1, args.steps
     rates, total_t = [], 0.0
-    for _ in range(5):
+    for _ in range(repeats):
         t = bo.sweep(MUEQ, reps=steps, nthreads=threads)
         total_t += t
         rates.append(nb * (HORIZON + 1) * steps / t)
     rates.sort()
-    v = rates[2]
+    v = rates[repeats // 2]
     assert bool((bo.status == 1).all())
     cpu = {"value": v, "unit": "knots/s", "cores": threads, "kind": "port",
-           "min": rates[0], "max": rates[-1], "repeats": 5,
-           "sample": "%d of %d instances per step, 5 repeats x %d steps (%.1f s in all), OpenMP over instances on %d "
+           "min": rates[0], "max": rates[-1], "repeats": repeats,
+           "sample": "%d of %d instances per step, %d repeat(s) x %d steps (%.1f s in all), OpenMP over instances on %d "
                      "threads (%d hardware threads visible; thread counts tried: %s), median of the repeats"
-                     % (nb, BATCH, steps, total_t, threads, avail, ", ".join("%d: %.1f ms/sweep" % (k, 1e3 * v_) for k, v_ in best.items()))}
+                     % (nb, BATCH, repeats, steps, total_t, threads, avail,
+                        ", ".join("%d: %.1f ms/sweep" % (k, 1e3 * v_) for k, v_ in best.items()))}
     if args.cpu_extra:
         try:
             cpu["single_instance"] = _single_instance_cpu_rows()
         except Exception as e:  # the extra rows never break the arm
             cpu["single_instance"] = "failed: %r" % (e,)
     line = {"metric": "riccati_knots_per_sec", "value": v, "unit": "knots/s", "n_gpus": args.gpus,
-            "steps": steps * 5, "warmup": nw, "ms_per_step": 1e3 * total_t / (5 * steps),
+            "steps": steps * repeats, "warmup": nw, "ms_per_step": 1e3 * total_t / (repeats * steps),
             "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f64",
             "data": "synthetic", "impl": "reference",
             "config": {"workload": WORKLOAD, "step_sample": "%d instances per step" % nb,
@@ -303,6 +308,40 @@ def parity_sample(gar, solver, stage, term, G0, g0, nsamp=16):
     return worst
 
 
+DUMP_BYTES = 60 * 10 ** 6  # the sample's data; with the .npy headers it stays below 64 MB
+DUMP_SEED = 2024
+
+
+def dump_outputs(gar, solver, outdir):
+    """Writes what the last sweep returned to its caller -- gains ff, fb, value function Vxx, vx, terminal
+    gains ffT, fbT and the primal-dual trajectory xs, us, vs, vsT, lbd0, lbdas -- as <outdir>/<name>.npy
+    (float64, Vxx indexed [b, t, i, j]), so that two builds can be compared output for output.  A full batch
+    is too large to keep: every array holds the same instances, a seeded sample of the batch (sorted, the
+    same for every build at a given batch size) as large as fits DUMP_BYTES in all; idx.npy holds their
+    batch indices (as float64)."""
+    import numpy as np
+    outs = {"ff": gar.OUT_FF, "fb": gar.OUT_FB, "Vxx": gar.OUT_VXX, "vx": gar.OUT_VX, "ffT": gar.OUT_FFT,
+            "fbT": gar.OUT_FBT, "xs": gar.OUT_XS, "us": gar.OUT_US, "vs": gar.OUT_VS, "vsT": gar.OUT_VST,
+            "lbd0": gar.OUT_LBD0, "lbdas": gar.OUT_LBDAS}
+    shapes = {k: solver.out_shape(w) for k, w in outs.items() if int(np.prod(solver.out_shape(w))) > 0}
+    B = solver.dims.batch
+    per_instance = sum(int(np.prod(s[1:])) for s in shapes.values()) * 8
+    n = max(1, min(B, DUMP_BYTES // per_instance))
+    idx = np.sort(np.random.default_rng(DUMP_SEED).choice(B, n, replace=False))
+    per_instance_outs = (gar.OUT_FFT, gar.OUT_FBT, gar.OUT_VST, gar.OUT_LBD0)
+    os.makedirs(outdir, exist_ok=True)
+    np.save(os.path.join(outdir, "idx.npy"), idx.astype(np.float64))
+    for name, shape in shapes.items():
+        knots = 1 if outs[name] in per_instance_outs else shape[1]
+        a = np.empty((n,) + tuple(shape[1:]))
+        for j, b in enumerate(idx):
+            solver.get_range_into(outs[name], int(b), 1, 0, knots, a[j], gar.AB2_HOST)
+        solver.synchronize()
+        if outs[name] == gar.OUT_VXX:  # column-major blocks in memory
+            a = a.transpose(0, 1, 3, 2)
+        np.save(os.path.join(outdir, name + ".npy"), np.ascontiguousarray(a))
+
+
 def bind_to_gpu_numa(local):
     """Pin this process to the CPUs closest to its GPU (NVML's ideal-CPU mask = the GPU's NUMA node)
     BEFORE any pinned host memory is allocated, so the e2e staging buffers land on that node (first
@@ -348,7 +387,13 @@ def main():
     ap.add_argument("--strong-legs", type=int, default=0, help="parallel-in-time legs for the strong-scaling run")
     ap.add_argument("--gather", default="peer", choices=["peer", "nccl"],
                     help="the one exchange: fused pack + NVLink peer-memory all-gather, or pack kernel + ncclAllGather")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the outputs of the last one as DIR/<name>.npy (rank 0's shard)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the product arm's outputs; --impl reference has none to write")
     if args.config != "c2":
         NX, NU, NC, NCT, HORIZON, BATCH, MUEQ, WORKLOAD = CONFIGS[args.config]
         if args.batch == 4096:
@@ -469,6 +514,8 @@ def main():
     ms_per_step = ms / args.steps
     knots = B * (N + 1) * world
     value = knots / (ms_per_step * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(gar, solver, args.dump_outputs)
 
     # ---- e2e through the C ABI with host (pinned) buffers ----
     e2e = None

@@ -61,9 +61,11 @@ def test_create_fails_loudly_without_cuda(lib):
 
 
 def test_unsupported_shape_is_an_error(lib):
+    """Refused before any device is touched, so the same error with or without a GPU
+    (57 x 28, BASELINE config 5, is a supported CTA-per-instance shape)."""
     import aligator_b200.gar as gar
-    with pytest.raises(gar.GarError):
-        gar.CudaRiccatiBatch(57, 28, 0, 0, 57, 10, 4)
+    with pytest.raises(gar.GarError, match="does not fit one CTA"):
+        gar.CudaRiccatiBatch(120, 40, 0, 0, 120, 10, 4)
 
 
 def test_product_does_not_import_oracle():
